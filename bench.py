@@ -2,6 +2,7 @@
 """bench.py -- scene-pairs/sec of the PointContrast hot path (Res16UNet34C + PointInfoNCE, 2.5 cm voxels).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--loss nce|hardest] [--workload c1|c0|c4]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one full training iteration on one batch of synthetic scene pairs per rank: coordinate-manager build for
@@ -25,6 +26,12 @@ count chosen by a measured sweep; it never loads libpcb200.so.
 
 --workload c4: BASELINE configs[4], S3DIS-shaped full-scene inference (5 cm voxels, eval-mode BatchNorm, 13 classes, forward only,
 `downstream/semseg/lib/test.py:95-117`); metric scenes/sec.
+
+--dump-outputs DIR: after the timed steps, what the last of them computed goes to DIR/<name>.npy, so that two builds can be compared
+output for output (inputs, weights and sampling draws are seeded: the same arguments give the same inputs).  Training workloads:
+loss (float64, the step's loss or (loss, pos, neg)), params and grads (the flat parameters after the step's SGD update and the
+step's gradients), bn_running_stats; c4: logits and pred of the last scene.  An array of more than 2^19 rows is a fixed seeded
+sample of 2^19 rows in ascending order (`host_rows`).
 """
 import argparse
 import json
@@ -60,7 +67,33 @@ def parse():
     ap.add_argument("--workload", default="c1", choices=list(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-json", default=None, help="write the per-launch conv profile of one step here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32 / float64, a fixed sample of large arrays)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_ROWS = 1 << 19     # rows kept of a larger output: <= 64 MB in all for every workload
+
+
+def host_rows(x, seed=0):
+    """`x` as a host array; with more than DUMP_ROWS rows, a fixed seeded sample of DUMP_ROWS of them in ascending order (the same
+    rows for any array of the same length)."""
+    if len(x) > DUMP_ROWS:
+        idx = np.sort(np.random.default_rng(seed).choice(len(x), DUMP_ROWS, replace=False))
+        x = x[torch.from_numpy(idx).to(x.device)]
+    return x.detach().cpu().numpy()
+
+
+def dump_outputs(dirname, arrays):
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(dirname, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
 
 
 def static_config(args, world):
@@ -322,6 +355,12 @@ def run_ours(args):
     clk = clocks.stop(t_wall0, t_wall1) if clocks else None
     pairs_per_step = wl["batch"] * world
     value = pairs_per_step * args.steps / (ms_total / 1e3)
+    outputs = None
+    if args.dump_outputs and rank == 0:    # the last timed step: its loss(es), the parameters it left, its gradients, BatchNorm statistics
+        opt = trainer.optimizer
+        outputs = {"loss": np.asarray(loss, dtype=np.float64).reshape(-1), "params": host_rows(opt.flat_param),
+                   "grads": host_rows(opt.flat_grad),
+                   "bn_running_stats": torch.cat([b.reshape(-1) for b in trainer.model.buffers() if b.dtype.is_floating_point]).cpu().numpy()}
 
     # ---- end-to-end through the public trainer call, host (pinned) batches
     it = iter(loader)
@@ -422,6 +461,8 @@ def run_ours(args):
                 "clocks": clk, "gpu_launches": int(launches),
                 "e2e": {"value": e2e_value, "unit": "pairs/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4},
                 "roofline": roof, "cpu_baseline": cb}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -441,24 +482,31 @@ def run_c4(args):
     devb = [(torch.from_numpy(s["feats"]).cuda(), torch.from_numpy(s["coords"]).cuda()) for s in scenes]
     host = [(torch.from_numpy(s["feats"]).pin_memory(), torch.from_numpy(s["coords"]).pin_memory()) for s in scenes]
 
+    last = {}
+
     def run(batches, n, to_host):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize(); e0.record()
         for i in range(n):
             f, c = batches[i % len(batches)]
             with torch.no_grad():
-                pred = net(me.SparseTensor(f, coords=c).to("cuda")).F.argmax(1)
+                logits = net(me.SparseTensor(f, coords=c).to("cuda")).F
+                pred = logits.argmax(1)
             if to_host:
                 pred = pred.cpu()
         e1.record(); torch.cuda.synchronize()
+        last.update(logits=logits, pred=pred)
         return e0.elapsed_time(e1) / n
-    run(devb, args.warmup, False)
+    if args.warmup:
+        run(devb, args.warmup, False)
     clocks = Clocks(0)
     t0 = time.time(); l0 = _lib.launch_count()
     ms = run(devb, args.steps, False)
     launches = _lib.launch_count() - l0
     t1 = time.time()
     clk = clocks.stop(t0, t1)
+    if args.dump_outputs:                  # the last timed scene: per-voxel class scores and the predicted class
+        dump_outputs(args.dump_outputs, {"logits": host_rows(last["logits"]), "pred": host_rows(last["pred"])})
     ms_e2e = run(host, args.steps, True)
     nvox = sum(len(s["coords"]) for s in scenes) / len(scenes)
     h2d = int(np.mean([f.numel() * 4 + c.numel() * 4 for f, c in host]))

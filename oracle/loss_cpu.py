@@ -3,7 +3,7 @@
 The reference draws its random subsets from process-global RNGs (`lib/ddp_trainer.py:199-200,203,404,413`).
 For parity the draws are *injected*: every function here takes the already-chosen indices.
 
-PINNED against the reference's own unmodified code (tests/test_oracle_reference.py, runs where /root/reference exists):
+PINNED against the reference's own unmodified code (tests/test_oracle_reference.py, against its outputs recorded in tests/golden/):
   * `hardest_contrastive_loss` == `HardestContrastiveLossTrainer.contrastive_hardest_negative_loss`
     (`lib/ddp_trainer.py:186-238`), same numpy RNG draws, rtol 1e-12;
   * `select_positives` + `point_nce_loss` == the loss and gradients of `PointNCELossTrainer._train_iter`

@@ -4,9 +4,9 @@ to the GPU box (where /root/reference does not exist) and be EXECUTED there, unm
     python oracle/stage_ref.py        (also run by __graft_entry__.build() in the build container)
 
 Copies `/root/reference/pretrain/pointcontrast/model/` (res16unet.py, resnet.py, modules/) byte for byte into
-`oracle/_ref/pointcontrast/model/`.  `oracle/_ref/` is git-ignored (never part of the history, like the built .so files)
-but not gpurun-ignored.  Nothing in the product path imports it; `tests/refload.py` does, for
-`tests/test_gpu_c1.py::test_reference_model_file_runs_on_cuda_fused`.  The reference's arithmetic layer (MinkowskiEngine
+`oracle/_ref/pointcontrast/model/`.  `oracle/_ref/` is git-ignored (never part of the history, like the built .so files).
+Nothing in the product path imports it; `tests/refload.py` does, for the CPU baseline of `bench.py` (the reference's model
+file on the oracle operators).  The reference's arithmetic layer (MinkowskiEngine
 0.4.3, C++/CUDA) is not under /root/reference, so there is nothing to compile (DESIGN.md "Oracle").
 """
 import os

@@ -7,8 +7,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-REFERENCE = "/root/reference"
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run with -m gpu on the B200 box)")
@@ -25,8 +23,3 @@ def pytest_collection_modifyitems(config, items):
     for it in items:
         if "gpu" in it.keywords:
             it.add_marker(skip)
-
-
-@pytest.fixture(scope="session")
-def have_reference():
-    return os.path.isdir(os.path.join(REFERENCE, "pretrain", "pointcontrast"))

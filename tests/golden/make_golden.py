@@ -1,8 +1,9 @@
-"""Generates tests/golden/c0_res16unet34c.npz  (run in the build container, where /root/reference exists):
+"""Generates tests/golden/c0_res16unet34c.npz and c0_res16unet34c_features.npz (run where the original project's
+`pretrain/pointcontrast` package can be imported, see tests/refload.py):
 
     python tests/golden/make_golden.py
 
-The REFERENCE's own model graph (`/root/reference/pretrain/pointcontrast/model/res16unet.py`, imported unmodified)
+The REFERENCE's own model graph (`pretrain/pointcontrast/model/res16unet.py` of the original project, imported unmodified)
 is executed on the CPU oracle (oracle/me_cpu.py, fp64) for BASELINE config C0: one synthetic scene pair (~4k voxels
 per view), Res16UNet34C, PointInfoNCE (T = 0.4, npos = 4096), deterministic weights (tests/helpers.det_init).
 Stored: the inputs, per-point output features of both views, the loss, the chosen positive indices, the gradient
@@ -67,9 +68,12 @@ def main():
                g_final=sd["final.kernel"].grad.numpy().astype(np.float32),
                g_b8=sd["block8.1.conv2.kernel"].grad.numpy()[13].astype(np.float32), bn_running_mean_l1=bn_rm,
                grad_relerr_f32=f32_err, feat_relerr_f32=np.float64(f32_feat_err))
-    path = os.path.join(ROOT, "tests", "golden", "c0_res16unet34c.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes; loss", loss.item(), "N0", len(batch["sinput0_C"]))
+    feats = {k: out.pop(k) for k in ("F0", "F1")}           # a file of their own: each file stays under 1 MB
+    for name, arrays in (("c0_res16unet34c.npz", out), ("c0_res16unet34c_features.npz", feats)):
+        path = os.path.join(ROOT, "tests", "golden", name)
+        np.savez_compressed(path, **arrays)
+        print("wrote", path, os.path.getsize(path), "bytes")
+    print("loss", loss.item(), "N0", len(batch["sinput0_C"]))
 
 
 if __name__ == "__main__":

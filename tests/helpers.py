@@ -1,9 +1,42 @@
 """Shared helpers for the parity tests."""
 import contextlib
+import json
 import math
+import os
 
 import numpy as np
 import torch
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def load_c0_golden():
+    """tests/golden/c0_res16unet34c.npz with the per-point features of tests/golden/c0_res16unet34c_features.npz, as one dict
+    (two files keep each under 1 MB)."""
+    g = dict(np.load(os.path.join(GOLDEN, "c0_res16unet34c.npz")))
+    g.update(np.load(os.path.join(GOLDEN, "c0_res16unet34c_features.npz")))
+    return g
+
+
+def model_structure(net):
+    """Module tree and state-dict layout of a Res16UNet built on any MinkowskiEngine-compatible module, as JSON data: every
+    module's name and class, a convolution's kernel offsets, stride and bias flag, a BatchNorm's momentum and eps."""
+    mods = []
+    for name, m in net.named_modules():
+        d = {"name": name, "class": type(m).__name__}
+        if getattr(m, "kernel_generator", None) is not None:
+            d.update(offsets=np.asarray(m.kernel_generator.offsets).tolist(), stride=[int(s) for s in m.stride], has_bias=bool(m.has_bias))
+        if isinstance(getattr(m, "bn", None), torch.nn.BatchNorm1d):
+            d.update(momentum=float(m.bn.momentum), eps=float(m.bn.eps))
+        mods.append(d)
+    return {"n_params": sum(p.numel() for p in net.parameters()), "modules": mods,
+            "state_dict": [[k, list(v.shape)] for k, v in net.state_dict().items()]}
+
+
+def reference_structure():
+    """`model_structure` of the original project's Res16UNet34C (tests/golden/make_reference_fixtures.py)."""
+    with open(os.path.join(GOLDEN, "reference_res16unet34c_structure.json")) as f:
+        return json.load(f)
 
 
 def rand_coords(rng, n, lo=-20, hi=21, batches=2):

@@ -16,10 +16,9 @@ import torch
 from oracle import loss_cpu
 from oracle import me_cpu as OR
 from tests import refload
-from tests.helpers import det_init, max_rel_err, model_backend, rel_err
+from tests.helpers import det_init, load_c0_golden, max_rel_err, model_backend, rel_err
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(__file__), "golden", "c0_res16unet34c.npz")
 
 
 def _grad_tol(floor, factor):
@@ -41,12 +40,13 @@ def _gpu_net(seed=0, normalize=True):
 
 def test_c0_against_reference_graph_golden():
     from pointcontrast_b200 import losses, me
-    g = np.load(GOLD)
+    g = load_c0_golden()
     net = _gpu_net(0)
     F = []
     for v in ("0", "1"):
         st = me.SparseTensor(torch.from_numpy(g["X" + v]), coords=torch.from_numpy(g["C" + v])).to("cuda")
         F.append(net(st).F)
+    assert "_fused_runner" in net.__dict__                  # a training-mode call takes the fused executor
     assert max_rel_err(F[0], torch.from_numpy(g["F0"])) < 1e-3 and max_rel_err(F[1], torch.from_numpy(g["F1"])) < 1e-3
     loss = losses.point_nce_loss(F[0], F[1], torch.from_numpy(g["q_rows"]).cuda(), torch.from_numpy(g["k_rows"]).cuda(), 0.4)
     assert abs(float(loss.detach()) - float(g["loss"])) / float(g["loss"]) < 1e-3

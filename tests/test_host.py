@@ -65,24 +65,19 @@ def test_offset_tables_match_oracle():
     assert [m.value for m in me.RegionType] == [0, 1, 2, 3]
 
 
-def test_own_model_matches_reference_model_structure(have_reference):
-    if not have_reference:
-        pytest.skip("/root/reference not present")
-    from pointcontrast_b200 import me
+def test_own_model_matches_reference_model_structure():
+    """This package's Res16UNet34C on its own MinkowskiEngine surface against the original model file's, as recorded in
+    tests/golden/reference_res16unet34c_structure.json: the same modules in the same order (classes, kernel offsets, strides,
+    biases, BatchNorm momentum / eps) and the same state-dict layout."""
     from pointcontrast_b200.model import load_model
-    cfg = refload.default_config()
-    net = load_model("Res16UNet34C")(3, 32, cfg, D=3)
-    ref = refload.load_reference_model_module(me.install).load_model("Res16UNet34C")(3, 32, cfg, D=3)
-    sd, rsd = net.state_dict(), ref.state_dict()
-    assert list(sd) == list(rsd) and all(sd[k].shape == rsd[k].shape for k in sd)
-    for (n1, m1), (n2, m2) in zip(net.named_modules(), ref.named_modules()):
-        assert n1 == n2
-        if isinstance(m1, me.MinkowskiConvolution) or isinstance(m1, me.MinkowskiConvolutionTranspose):
-            assert type(m1) is type(m2) and (m1.kernel_generator.offsets == m2.kernel_generator.offsets).all()
-            assert m1.stride == m2.stride and m1.has_bias == m2.has_bias
-        if isinstance(m1, me.MinkowskiBatchNorm):
-            assert m1.bn.momentum == m2.bn.momentum and m1.bn.eps == m2.bn.eps
-    assert sum(p.numel() for p in net.parameters()) == 37_847_808
+    from tests.helpers import model_structure, reference_structure
+    net = load_model("Res16UNet34C")(3, 32, refload.default_config(), D=3)
+    own, ref = model_structure(net), reference_structure()
+    assert own["state_dict"] == ref["state_dict"]
+    assert [m["name"] for m in own["modules"]] == [m["name"] for m in ref["modules"]]
+    for m1, m2 in zip(own["modules"], ref["modules"]):
+        assert m1 == m2, m1["name"]
+    assert own["n_params"] == ref["n_params"] == 37_847_808
 
 
 def test_no_cpu_compute_path():
@@ -109,8 +104,8 @@ def test_product_code_never_imports_the_oracle():
 
 def test_golden_fixture_is_consistent_with_the_oracle():
     """The committed golden file replays on the oracle with THIS repo's model wiring (own graph == reference graph)."""
-    from tests.helpers import det_init, max_rel_err, model_backend
-    g = np.load(os.path.join(ROOT, "tests", "golden", "c0_res16unet34c.npz"))
+    from tests.helpers import det_init, load_c0_golden, max_rel_err, model_backend
+    g = load_c0_golden()
     with model_backend(OR) as mod:
         net = mod.Res16UNet34C(3, 32, refload.default_config(), D=3)
         det_init(net, 0)                   # fp32 parameter values (what the GPU model holds), evaluated in fp64

@@ -1,37 +1,20 @@
-"""Runs the reference's own Python (model graph, hardest-contrastive loss) on the oracle.  Needs /root/reference."""
+"""The oracle against the original PointContrast code: its model graph and its two losses, as recorded from that code in
+tests/golden/ by tests/golden/make_reference_fixtures.py."""
+import os
+import types
+
 import numpy as np
-import pytest
 import torch
 
 from oracle import loss_cpu, me_cpu
 from tests import refload
+from tests.helpers import GOLDEN, model_backend, model_structure, reference_structure
 
-pytestmark = pytest.mark.skipif(not refload.available(), reason="/root/reference not present")
-
-
-def test_reference_res16unet34c_builds_on_oracle():
-    model_pkg = refload.load_reference_model_module(me_cpu.install)
-    Net = model_pkg.load_model("Res16UNet34C")
-    net = Net(3, 32, refload.default_config(), D=3)
-    n = sum(p.numel() for p in net.parameters())
-    assert n == 37_847_808
-    convs = [m for m in net.modules() if isinstance(m, me_cpu.MinkowskiConvolution)]
-    trs = [m for m in net.modules() if isinstance(m, me_cpu.MinkowskiConvolutionTranspose)]
-    bns = [m for m in net.modules() if isinstance(m, me_cpu.MinkowskiBatchNorm)]
-    assert (len(convs), len(trs), len(bns)) == (59, 4, 62)
-    moms = sorted(m.bn.momentum for m in bns)
-    assert moms.count(0.1) == 46 and moms.count(0.05) == 16          # SURVEY 8a row B1
-    sd = net.state_dict()
-    assert sd["conv0p1s1.kernel"].shape == (27, 3, 32)
-    assert sd["final.kernel"].shape == (1, 96, 32) and sd["final.bias"].shape == (1, 32)
-    assert sd["block2.0.downsample.0.kernel"].shape == (1, 32, 64)
-    assert "bn0.bn.running_mean" in sd and "block8.1.norm2.bn.weight" in sd
+HARDEST_NUM_POS = (1024, 5000)
+NCE_NPOS = (64, 1 << 20)                             # with and without the npos subsample (`lib/ddp_trainer.py:411-415`)
 
 
-def test_hardest_loss_oracle_matches_reference_function():
-    tr = refload.load_reference_trainer_module(me_cpu.install)
-    obj = tr.HardestContrastiveLossTrainer.__new__(tr.HardestContrastiveLossTrainer)
-    obj.pos_thresh, obj.neg_thresh = 0.1, 1.4
+def hardest_inputs():
     g = torch.Generator().manual_seed(0)
     N0, N1, P = 700, 650, 3000
     F0 = torch.nn.functional.normalize(torch.randn(N0, 32, generator=g, dtype=torch.float64), dim=1)
@@ -40,9 +23,56 @@ def test_hardest_loss_oracle_matches_reference_function():
     rng = np.random.default_rng(0)
     i0 = np.sort(rng.integers(0, 300, P))
     pairs = torch.from_numpy(np.stack([i0, np.clip(i0 + rng.integers(-1, 2, P), 0, N1 - 1)], 1))
-    for num_pos in (1024, 5000):
-        np.random.seed(7)
-        ref_pos, ref_neg = obj.contrastive_hardest_negative_loss(F0, F1, pairs, num_pos=num_pos, num_hn_samples=256)
+    return F0, F1, pairs
+
+
+class StandIn(torch.nn.Module):
+    """Stand-in for Res16UNet in the PointInfoNCE check: per-row features from (feats, coords)."""
+    def __init__(self):
+        super().__init__()
+        torch.manual_seed(0)
+        self.lin = torch.nn.Linear(7, 32).double()
+
+    def forward(self, s):
+        x = torch.cat([s.F.double(), torch.sin(s.C.double() * 0.37)], 1)
+        return types.SimpleNamespace(F=torch.nn.functional.normalize(self.lin(x), dim=1))
+
+
+def nce_batch():
+    from pointcontrast_b200 import synth
+    return synth.collate_pairs([synth.synth_pair(3, scale=0.1), synth.synth_pair(4, scale=0.1)])
+
+
+def _recorded():
+    return np.load(os.path.join(GOLDEN, "reference_losses.npz"))
+
+
+def test_reference_res16unet34c_builds_on_oracle():
+    """The original Res16UNet34C as recorded on the oracle, and this package's model file built on the oracle: the same modules,
+    kernel offsets, strides, BatchNorm settings and state-dict layout."""
+    ref = reference_structure()
+    assert ref["n_params"] == 37_847_808
+    classes = [m["class"] for m in ref["modules"]]
+    assert (classes.count("MinkowskiConvolution"), classes.count("MinkowskiConvolutionTranspose"),
+            classes.count("MinkowskiBatchNorm")) == (59, 4, 62)
+    moms = sorted(m["momentum"] for m in ref["modules"] if m["class"] == "MinkowskiBatchNorm")
+    assert moms.count(0.1) == 46 and moms.count(0.05) == 16          # SURVEY 8a row B1
+    sd = dict((k, tuple(s)) for k, s in ref["state_dict"])
+    assert sd["conv0p1s1.kernel"] == (27, 3, 32)
+    assert sd["final.kernel"] == (1, 96, 32) and sd["final.bias"] == (1, 32)
+    assert sd["block2.0.downsample.0.kernel"] == (1, 32, 64)
+    assert "bn0.bn.running_mean" in sd and "block8.1.norm2.bn.weight" in sd
+    with model_backend(me_cpu) as mod:
+        net = mod.Res16UNet34C(3, 32, refload.default_config(), D=3)
+    assert model_structure(net) == ref
+
+
+def test_hardest_loss_oracle_matches_reference_function():
+    rec = _recorded()
+    F0, F1, pairs = hardest_inputs()
+    N0, N1, P = len(F0), len(F1), len(pairs)
+    for num_pos in HARDEST_NUM_POS:
+        ref_pos, ref_neg = (torch.tensor(v, dtype=torch.float64) for v in rec[f"hardest_{num_pos}"])
         np.random.seed(7)
         sel0 = np.random.choice(N0, 256, replace=False)
         sel1 = np.random.choice(N1, 256, replace=False)
@@ -51,54 +81,25 @@ def test_hardest_loss_oracle_matches_reference_function():
         assert torch.allclose(pos, ref_pos, rtol=1e-12) and torch.allclose(neg, ref_neg, rtol=1e-12)
 
 
-def test_point_nce_oracle_matches_reference_train_iter(monkeypatch):
-    """Rows L1 + L2: the reference's own `PointNCELossTrainer._train_iter` (`lib/ddp_trainer.py:380-440`, unmodified,
-    `NCESoftmaxLoss` from `lib/criterion.py`) run on the CPU -- its hard-coded `.cuda()` calls patched to identity, a small
-    stand-in model -- against `loss_cpu.select_positives` + `point_nce_loss` fed with the same RNG draws."""
-    import types
-    tr = refload.load_reference_trainer_module(me_cpu.install)
-    monkeypatch.setattr(torch.Tensor, "cuda", lambda self, *a, **k: self)
-    monkeypatch.setattr(torch.nn.Module, "cuda", lambda self, *a, **k: self)
-
-    class Net(torch.nn.Module):                      # stand-in for Res16UNet: per-row features from (feats, coords)
-        def __init__(self):
-            super().__init__()
-            torch.manual_seed(0)
-            self.lin = torch.nn.Linear(7, 32).double()
-
-        def forward(self, s):
-            x = torch.cat([s.F.double(), torch.sin(s.C.double() * 0.37)], 1)
-            return types.SimpleNamespace(F=torch.nn.functional.normalize(self.lin(x), dim=1))
-
-    from pointcontrast_b200 import synth
-    batch = synth.collate_pairs([synth.synth_pair(3, scale=0.1), synth.synth_pair(4, scale=0.1)])
+def test_point_nce_oracle_matches_reference_train_iter():
+    """Rows L1 + L2: the original `PointNCELossTrainer._train_iter` (`lib/ddp_trainer.py:380-440`, `NCESoftmaxLoss` from
+    `lib/criterion.py`) run on the CPU with a small stand-in model -- its loss and the stand-in's weight gradient, recorded --
+    against `loss_cpu.select_positives` + `point_nce_loss` fed with the same RNG draws."""
+    rec = _recorded()
+    batch = nce_batch()
     inp = {k: (torch.from_numpy(v) if isinstance(v, np.ndarray) else v) for k, v in batch.items()}
-    inp["pcd0"], inp["pcd1"] = inp["sinput0_C"], inp["sinput1_C"]                  # only .shape[0] is read (`:400`)
     nq = len(np.unique(batch["correspondences"][:, 0]))
-
-    class It:
-        def next(self):
-            return inp
-
-    for npos in (64, 1 << 20):                       # with and without the npos subsample (`:411-415`)
-        net = Net()
-        obj = tr.PointNCELossTrainer.__new__(tr.PointNCELossTrainer)
-        obj.model, obj.cur_device, obj.T, obj.npos = net, "cpu", 0.4, npos
-        obj.optimizer = types.SimpleNamespace(zero_grad=lambda: None, step=lambda: None)
-        obj.config = refload.Cfg(misc=dict(num_gpus=1))
-        torch.manual_seed(11); np.random.seed(12)
-        ref_loss = obj._train_iter(It(), [tr.AverageMeter(), tr.Timer(), tr.Timer()])
-        ref_grad = net.lin.weight.grad.clone()
-        # the oracle with the same draws
+    for npos in NCE_NPOS:
+        ref_loss, ref_grad = float(rec[f"nce_{npos}_loss"]), torch.from_numpy(rec[f"nce_{npos}_grad"])
         torch.manual_seed(11); np.random.seed(12)
         uniform = torch.distributions.Uniform(0, 1).sample([nq])
         sampled = np.random.choice(nq, npos, replace=False) if npos < nq else None
-        net2 = Net()
-        F0 = net2(me_cpu.SparseTensor(inp["sinput0_F"], coords=inp["sinput0_C"])).F
-        F1 = net2(me_cpu.SparseTensor(inp["sinput1_F"], coords=inp["sinput1_C"])).F
+        net = StandIn()
+        F0 = net(me_cpu.SparseTensor(inp["sinput0_F"], coords=inp["sinput0_C"])).F
+        F1 = net(me_cpu.SparseTensor(inp["sinput1_F"], coords=inp["sinput1_C"])).F
         q, k = loss_cpu.select_positives(batch["correspondences"], uniform, npos, sampled)
         assert len(q) == min(npos, nq)
         loss = loss_cpu.point_nce_loss(F0, F1, q, k, 0.4)
         loss.backward()
         assert abs(float(loss) - ref_loss) < 1e-12 * abs(ref_loss), (float(loss), ref_loss)
-        assert torch.allclose(net2.lin.weight.grad, ref_grad, rtol=1e-10, atol=1e-14)
+        assert torch.allclose(net.lin.weight.grad, ref_grad, rtol=1e-10, atol=1e-14)
