@@ -282,6 +282,19 @@ int pcb_nce_forward_backward(const float* q, const float* k, int64_t n, int D, f
 size_t pcb_ce_ws_bytes(int64_t n);
 int pcb_ce_forward_backward(const float* logits, const int64_t* target, int64_t n, int C, int64_t ignore_index, float grad_scale,
                             float* loss, float* dlogits, void* ws, size_t ws_bytes, void* stream);
+/* Semantic-segmentation metrics of one batch (`downstream/semseg/lib/test.py:119-149`, `lib/utils.py:117-133`) on logits [n, C]
+ * (contiguous fp32) and int64 targets.  A row is valid when 0 <= target < C and target != ignore_index; the others count in no loss,
+ * precision or histogram term and are negatives for every class in the average precision.
+ *   pred  [n] int32: first maximal index of each row (may be NULL)
+ *   hist  [C*C] int64, ACCUMULATED (+=): hist[target * C + pred] over the valid rows
+ *   stats [4] fp64 = {sum of the cross-entropy over the valid rows, #valid, #(pred == target) among them, n}
+ *   ap    [C] fp64: uninterpolated average precision of softmax column c against target == c, equal scores ranked as one group;
+ *         NaN for a class without a positive row
+ *   prob  [n, C] fp32: the softmax the average precision ranked by (may be NULL)
+ * 2 <= C <= 64, n >= 1, n * C < 2^31.  ws: pcb_seg_eval_ws_bytes(n, C).  Deterministic: repeated calls give bit-identical stats / ap. */
+size_t pcb_seg_eval_ws_bytes(int64_t n, int C);
+int pcb_seg_eval(const float* logits, const int64_t* target, int64_t n, int C, int64_t ignore_index, int32_t* pred, int64_t* hist,
+                 double* stats, double* ap, float* prob, void* ws, size_t ws_bytes, void* stream);
 /* Row-wise L2 normalisation of the output features, y = x / ||x||_2 with no epsilon (`model/res16unet.py:262-266`), and its
  * backward dx = (dy - y (y.dy)) / ||x||.  inv_norm: [n] scratch written by forward, read by backward. */
 int pcb_l2norm_forward(const float* X, int64_t n, int C, float* Y, float* inv_norm, void* stream);

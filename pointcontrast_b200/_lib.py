@@ -70,6 +70,8 @@ _SIGS = {
     "pcb_sgd_step": (_i, [_p, _p, _p, _l, _f, _f, _f, _f, _i, _f, _p]),
     "pcb_ce_ws_bytes": (_sz, [_l]),
     "pcb_ce_forward_backward": (_i, [_p, _p, _l, _i, _l, _f, _p, _p, _p, _sz, _p]),
+    "pcb_seg_eval_ws_bytes": (_sz, [_l, _i]),
+    "pcb_seg_eval": (_i, [_p, _p, _l, _i, _l, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "pcb_profile_enable": (_i, [_i]),
     "pcb_profile_read": (_i, [_p, _p, _i, C.POINTER(C.c_int)]),
     "pcb_unit_ws_bytes": (_sz, [_i, _l, _l, _i, _i]),

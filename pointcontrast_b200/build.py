@@ -10,7 +10,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
-SOURCES = ["coords.cu", "voxel.cu", "conv.cu", "conv_tc5.cu", "bn.cu", "loss.cu", "nce_tc5.cu", "unit.cu"]
+SOURCES = ["coords.cu", "voxel.cu", "conv.cu", "conv_tc5.cu", "bn.cu", "loss.cu", "nce_tc5.cu", "unit.cu", "seg_eval.cu"]
 OUT = os.path.join(HERE, "libpcb200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--threads", "4",

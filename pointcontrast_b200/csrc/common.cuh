@@ -69,6 +69,19 @@ inline void launch_kernel(void (*kernel)(Exp...), dim3 grid, dim3 block, size_t 
   cudaLaunchKernelEx(&cfg, kernel, static_cast<Act&&>(args)...);       // errors surface through check_launch (cudaGetLastError)
 }
 
+// Logsumexp of a row of C fp32 values shared by W lanes of a warp (lane strides by W; W = 32: one warp per row, W = 1: one thread per
+// row): m = max, s = sum of exp(x - m), returns m + log(s).  The cross-entropy (loss.cu) and segmentation-metric (seg_eval.cu) rows.
+template <int W>
+__device__ __forceinline__ float row_logsumexp(const float* __restrict__ x, int C, int lane, float& m, float& s) {
+  m = -INFINITY;
+  for (int c = lane; c < C; c += W) m = fmaxf(m, x[c]);
+  for (int o = W / 2; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  s = 0.f;
+  for (int c = lane; c < C; c += W) s += expf(x[c] - m);
+  for (int o = W / 2; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  return m + logf(s);
+}
+
 inline int current_device() { int dev = 0; cudaGetDevice(&dev); return (dev >= 0 && dev < 64) ? dev : 0; }
 
 inline int num_sms() {

@@ -299,14 +299,9 @@ __global__ void ce_rows_kernel(const float* __restrict__ X, const int64_t* __res
   const int64_t row = blockIdx.x * (int64_t)(blockDim.x >> 5) + (threadIdx.x >> 5);
   if (row >= n) return;
   const int64_t t = target[row];
-  float m = -INFINITY;
-  for (int c = lane; c < C; c += 32) m = fmaxf(m, X[row * C + c]);
-  for (int o = 16; o; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
-  float s = 0.f;
-  for (int c = lane; c < C; c += 32) s += expf(X[row * C + c] - m);
-  for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  float m, s;
+  const float lse = row_logsumexp<32>(X + row * C, C, lane, m, s);
   if (lane == 0) {
-    const float lse = m + logf(s);
     rowlse[row] = lse;
     rowloss[row] = (t == ignore || t < 0 || t >= C) ? 0.f : lse - X[row * C + t];
   }
